@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the tensegrity hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference] [--dump-outputs bench_outputs]
 
 A "step" is one env step (frame_skip = 20 substeps + obs/reward/done, in-kernel auto reset) of ALL envs of a
 rank: flat-ground XML, tr_env `straight`, fp64, uniform random ctrl in [-0.45, -0.15] drawn on the device
@@ -13,6 +13,8 @@ launching stream), max over ranks; `e2e` = the same through the public host API 
 obs/reward/done out, copies inside the timed region); `roofline` / `cpu_baseline` per the round contract.
 `--impl reference` times the CPU restatement of the reference path (the oracle; MuJoCo itself is not
 installable here) on all host threads -- rank 0 only.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (obs, reward, done) as .npy files, so that
+two builds run with the same arguments (identical seeded inputs) can be compared output for output.
 """
 import argparse
 import json
@@ -29,6 +31,7 @@ METRIC = "env-steps/sec (whole box, device-timed)"
 UNIT = "env-steps/s"
 CTRL_LO, CTRL_HI = -0.45, -0.15
 L2_BYTES = 126 * 2 ** 20
+DUMP_BYTES = 64 * 2 ** 20
 
 
 def algorithmic_bytes(obs_dim):
@@ -115,6 +118,23 @@ def run_reference(args, rank):
     }))
 
 
+def dump_outputs(out_dir, obs, rew, done):
+    """obs / reward (float64) and done (float32) of one step as DIR/<name>.npy, with env_index.npy naming the env of
+    each row: every env when that fits in DUMP_BYTES, else a fixed seeded sample of envs in ascending order."""
+    import numpy as np
+    import torch
+    n = obs.shape[0]
+    row_bytes = (obs.shape[1] + 2) * 8 + 4           # obs, reward, env_index in float64; done in float32
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+    idx = torch.as_tensor(rows, device=obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("obs", obs), ("reward", rew), ("done", done.float())):
+        np.save(os.path.join(out_dir, name + ".npy"), t[idx].cpu().numpy())
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+
+
 def cpu_baseline_sample(seconds=12.0):
     from oracle import oracle as O
     threads = O.lib().tsgo_max_threads()
@@ -145,7 +165,13 @@ def main():
     ap.add_argument("--sweep", default="4096,65536", help="extra env counts timed briefly at N=1 (reported in config)")
     ap.add_argument("--settle", type=int, default=200, help="untimed env steps between the reset and the timed window")
     ap.add_argument("--no-workloads", action="store_true", help="skip the policy-rollout sub-results (BASELINE configs[2], [3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write obs / reward / done of the last timed step (rank 0's envs) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -229,6 +255,8 @@ def main():
         sampler.start()
     ms, launches, stats = timed_run(env, n, args.steps, args.warmup, flush)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # env.obs / reward / done still hold the last timed step's results
+        dump_outputs(args.dump_outputs, env.obs, env.reward, env.done)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

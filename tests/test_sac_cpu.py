@@ -3,7 +3,6 @@ independent numpy restatement, target update, checkpoint layout, a toy learning 
 real simulator) is tests/test_gpu_sac.py."""
 import io
 import math
-import os
 import zipfile
 
 import numpy as np
@@ -12,8 +11,6 @@ import torch
 
 from tensegrity_rl_b200.sac import ReplayBuffer, SACLearner
 from tensegrity_rl_b200.spaces import Box
-
-REF_ZIP = "/root/reference/best_models_pretrained/forward/SAC_5500000.zip"
 
 
 def test_replay_ring_and_sampling():
@@ -125,19 +122,6 @@ def test_checkpoint_layout_and_roundtrip(tmp_path):
     torch.manual_seed(1); L2.update(1)
     for a, b in zip(L.policy.parameters(), L2.policy.parameters()):
         assert torch.allclose(a, b, atol=1e-6)
-
-
-@pytest.mark.skipif(not os.path.isfile(REF_ZIP), reason="reference checkpoints are only mounted in the build container")
-def test_resume_from_reference_checkpoint():
-    """run.py:44 `SAC.load(starting_point, env, ...)`: the reference's own zips load completely (weights, critics,
-    entropy coefficient, Adam moments, counters) and our actor agrees with the rollout-side loader."""
-    from tensegrity_rl_b200.policy import SacActor
-    L = SACLearner(39, 6, action_low=-0.45, action_high=-0.15, device="cpu").load_sb3_zip(REF_ZIP)
-    assert L.num_timesteps == 5_500_000 and L.n_updates == 5_499_900
-    assert float(L.log_ent_coef) == pytest.approx(-4.98975, abs=1e-4)
-    assert float(L.actor_opt.state_dict()["state"][0]["step"]) == 5_499_900
-    o = torch.randn(64, 39)
-    assert torch.allclose(SacActor(REF_ZIP, device="cpu")(o, deterministic=True), L.act(o, deterministic=True)[1], atol=1e-6)
 
 
 class _Bandit:
