@@ -12,9 +12,9 @@
 using namespace tb;
 
 // Production configuration (profiles/): three lanes per env, ten envs per warp, TB_WARPS warps per CTA and
-// TB_MIN_CTAS CTAs per SM (the register cap follows: 65536 / (TB_MIN_CTAS * TB_WARPS * 32) per thread).  TB_ALIGN: the
-// warps of a CTA walk through an env step in phase (CTA barriers at every substep and Newton iteration), so that they
-// share fetched instructions.
+// TB_MIN_CTAS CTAs per SM (the register cap follows: 65536 / (TB_MIN_CTAS * TB_WARPS * 32) per thread).  The step
+// kernel runs its warps aligned: the warps of a CTA walk through an env step in phase (CTA barriers at every substep
+// and Newton iteration), so that they share fetched instructions.
 #ifndef TB_MIN_CTAS
 #define TB_MIN_CTAS 1
 #endif
@@ -26,9 +26,6 @@ using namespace tb;
 #endif
 #ifndef TB_EPW_SMALL
 #define TB_EPW_SMALL 10    // envs per warp in that shape (fewer envs per warp = fewer envs waiting for the slowest one)
-#endif
-#ifndef TB_ALIGN
-#define TB_ALIGN 1
 #endif
 
 static_assert(STATE_STRIDE == TSG_STATE_STRIDE && INFO_DIM == TSG_INFO_DIM && NDRAW == TSG_NDRAW, "ABI constants");
@@ -84,7 +81,7 @@ __global__ void __launch_bounds__(W * 32, TB_MIN_CTAS) tb_env_kernel(const Model
     if (round >= env_rounds + pool_rounds) break;
     if (round < env_rounds) {
       const int first = (round * W + warp) * E;   // may lie beyond the batch: the warp then idles in step
-      if (MODE == MODE_STEP) run_step(S, m, c, io, L, first, TB_ALIGN != 0);
+      if (MODE == MODE_STEP) run_step(S, m, c, io, L, first, true);
       else if (MODE == MODE_RESET) run_reset(S, m, c, io, L, first);
       else run_forward(S, m, c, io, L, first);
     } else run_pool(S, m, c, io, L, ((round - env_rounds) * W + warp) * E, MODE == MODE_RESET);
