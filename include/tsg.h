@@ -43,6 +43,16 @@ typedef struct TsgHandle TsgHandle;
 #define TSG_PRECISION_F64 0 /* the reference's arithmetic (MuJoCo is float64); the default */
 #define TSG_PRECISION_F32 1 /* optional fp32 physics (state records, rewards and observations stay f64) */
 
+/* per-env parameter row (doubles, absolute values in model units); the nominal row holds the TsgModel fields of the
+ * same names */
+#define TSG_NPARAM 41
+#define TSG_PARAM_TEN_STIFFNESS 0    /* 9 */
+#define TSG_PARAM_TEN_DAMPING 9      /* 9 */
+#define TSG_PARAM_TEN_LENGTHSPRING 18 /* 18: lower, upper of tendon 0, then tendon 1, ... */
+#define TSG_PARAM_ACT_GAIN 36        /* 1 */
+#define TSG_PARAM_ACT_BIAS 37        /* 3 */
+#define TSG_PARAM_ACT_DYNPRM0 40     /* 1 */
+
 /* info row layout (doubles) */
 #define TSG_INFO_REW_FWD 0
 #define TSG_INFO_REW_CTRL 1
@@ -148,6 +158,29 @@ int tsg_get_heading_host(TsgHandle *h, double *heading);
 int tsg_set_heading_host(TsgHandle *h, const double *heading);
 /* last reset draws [n_envs][TSG_NDRAW], HOST buffer */
 int tsg_get_draws_host(TsgHandle *h, double *draws);
+
+/* Per-env tendon and actuator parameters (domain randomisation, system identification).  Every env record and every
+ * pool slot has a row of TSG_NPARAM doubles (TSG_PARAM_*) that replaces the model's ten_stiffness, ten_damping,
+ * ten_lengthspring, act_gain, act_bias and act_dynprm0 for that env.  Until one of the two setters is called a handle
+ * runs the model's constants; the first call gives every row the nominal row and switches the handle to the per-env
+ * kernels for good.
+ *
+ * tsg_set_param_ranges: HOST arrays lo, hi [TSG_NPARAM] of scale factors.  From then on every reset (tsg_reset, the
+ * synchronous auto-reset of tsg_step, and a pool slot's restart) draws a new row nominal[i] * U(lo[i], hi[i]).  The
+ * draws are Philox(seed ^ key, stream, (reset count << 8) | k) with the stream ids of the reset draws (env id, or
+ * 2^40 + slot id), so sharded handles reproduce an unsharded one.  Rules: finite, 0 <= lo <= hi, an act_dynprm0
+ * scale above 0; the lower and upper lengthspring of a tendon share one draw and need equal ranges.  lo = hi = NULL
+ * stops the draws (rows then stay as they are at resets).  Synchronises the device.
+ *
+ * tsg_set_env_params: explicit rows [n_envs][TSG_NPARAM] (DEVICE) for the envs whose mask byte is non-zero (NULL =
+ * all), in effect from the next launch on the stream; with ranges set they last until the env's next reset.  Fails on
+ * a handle with a reset pool: an env that receives a pool slot takes the row the slot was warmed up with.
+ *
+ * tsg_get_env_params: every env's row [n_envs][TSG_NPARAM] (DEVICE).  A checkpoint of env state is records + heading
+ * rings + parameter rows. */
+int tsg_set_param_ranges(TsgHandle *h, const double *lo, const double *hi);
+int tsg_set_env_params(TsgHandle *h, const double *params_dev, const uint8_t *mask_dev, void *stream);
+int tsg_get_env_params(TsgHandle *h, double *params_dev, void *stream);
 
 /* the calls behind the reference-shaped single env (envs.py tr_env / tensegrity_env: run.py:119,138): host buffers
  * in, host buffers out,

@@ -32,8 +32,12 @@ constexpr int ZONE_TOP = 0, ZONE_BOTTOM = 1, ZONE_MIDDLE = 2;
 // Arithmetic of a build.  `real`: kinematics, tendons, collision, integration.  `sreal`: the constraint solver (contact
 // rows, Newton Hessian, line search) -- the contact stiffness spans 1e6 x the bar inertia, so the solve needs fp64 to
 // stay within 1e-4 of the reference (pure fp32 lands at 1e-3 .. 1e-2: measured with the emulator, DESIGN.md).
-struct P64 { typedef double real; typedef double sreal; };
-struct P32 { typedef float real; typedef double sreal; };   // the optional fp32 mode: fp32 geometry, fp64 solver
+struct P64 { typedef double real; typedef double sreal; static constexpr bool per_env = false; };
+struct P32 { typedef float real; typedef double sreal; static constexpr bool per_env = false; };   // the optional fp32 mode: fp32 geometry, fp64 solver
+// The per-env-parameter variant of a build: the tendon and actuator constants come from the env's row of per-env
+// parameters in global memory (NPARAM doubles, PRM_* in tb_model.h) instead of the model.  A separate instantiation,
+// so that the kernels of handles without per-env parameters stay exactly what they are.
+template <typename B> struct PerEnv : B { static constexpr bool per_env = true; };
 
 // one contact.  Written by its owner lane; read by the lanes of the bars it touches.
 template <typename real>
@@ -51,9 +55,11 @@ struct Con {
   int zone, owner;     // owner: lane (bar index) that processes the contact, -1 = empty slot
 };
 
-// per-env slice of shared memory
+// per-env slice of shared memory; the per-env variant also holds the address of the env's parameter row
+template <bool PE> struct EnvShRow {};
+template <> struct EnvShRow<true> { const double* prm; };
 template <typename P>
-struct EnvSh {
+struct EnvSh : EnvShRow<P::per_env> {
   typedef typename P::real real;
   typedef typename P::sreal sreal;
   // world-frame exchange, rewritten by every pass; xpos / xmat / sph / tlen double as the "stale" kinematics the
@@ -632,6 +638,41 @@ TB_FN void kinematics(BarState<P>& B, EnvSh<P>& S, const ModelT<typename P::real
   }
 }
 
+// Tendon and actuator constants of the per-env variant, read from the env's row with the (real) cast make_model uses,
+// so that the nominal row reproduces the model bit for bit.  Plain loads, not __ldg: a reset writes the row in the
+// same launch (run_reset, run_pool).  The accessors hand the default variant the model's fields, read where the code
+// always read them.
+template <typename P> struct PrmRow { typename P::real tk, tdamp, tls[2], gain, bias[3], dynprm0; };
+template <typename P> TB_FN void load_act_prm(PrmRow<P>& R, const double* r) {
+  typedef typename P::real real;
+  R.gain = (real)r[PRM_GAIN];
+  for (int k = 0; k < 3; k++) R.bias[k] = (real)r[PRM_BIAS + k];
+  R.dynprm0 = (real)r[PRM_DYNPRM0];
+}
+template <typename P> TB_FN void load_ten_prm(PrmRow<P>& R, const double* r, int t) {
+  typedef typename P::real real;
+  R.tk = (real)r[PRM_TK + t]; R.tdamp = (real)r[PRM_TDAMP + t];
+  R.tls[0] = (real)r[PRM_TLS + 2 * t]; R.tls[1] = (real)r[PRM_TLS + 2 * t + 1];
+}
+template <typename P> TB_FN typename P::real prm_tk(const PrmRow<P>& R, const ModelT<typename P::real>& m, int t) {
+  if constexpr (P::per_env) return R.tk; else return m.tk[t];
+}
+template <typename P> TB_FN typename P::real prm_tdamp(const PrmRow<P>& R, const ModelT<typename P::real>& m, int t) {
+  if constexpr (P::per_env) return R.tdamp; else return m.tdamp[t];
+}
+template <typename P> TB_FN typename P::real prm_tls(const PrmRow<P>& R, const ModelT<typename P::real>& m, int t, int k) {
+  if constexpr (P::per_env) return R.tls[k]; else return m.tls[t][k];
+}
+template <typename P> TB_FN typename P::real prm_gain(const PrmRow<P>& R, const ModelT<typename P::real>& m) {
+  if constexpr (P::per_env) return R.gain; else return m.gain;
+}
+template <typename P> TB_FN typename P::real prm_bias(const PrmRow<P>& R, const ModelT<typename P::real>& m, int k) {
+  if constexpr (P::per_env) return R.bias[k]; else return m.bias[k];
+}
+template <typename P> TB_FN typename P::real prm_dynprm0(const PrmRow<P>& R, const ModelT<typename P::real>& m) {
+  if constexpr (P::per_env) return R.dynprm0; else return m.dynprm0;
+}
+
 // tendons: length, velocity, spring-damper / actuator force; then qacc_smooth, the world-frame inertia, and the damping
 // block Dblk of the bar (for implicitfast)
 template <typename P>
@@ -643,9 +684,12 @@ TB_FN void smooth_dynamics(BarState<P>& B, EnvSh<P>& S, const ModelT<typename P:
   const real* Mb = m.M + 6 * b;
   real f[6] = {0, 0, 0, 0, 0, 0};
   for (int e = 0; e < 21; e++) Dblk[e] = 0;
+  PrmRow<P> R;
+  if constexpr (P::per_env) load_act_prm(R, S.prm);
   TB_UNROLL1
   for (int n = 0; n < m.nends[b]; n++) {
     const int end = m.ends[b][n], t = end >> 1, s = end & 1, oe = end ^ 1, ob = m.tbody[oe];
+    if constexpr (P::per_env) load_ten_prm(R, S.prm, t);
     real pown[3], poth[3], dir[3];
     copy3(pown, S.u.site + 3 * end); copy3(poth, S.u.site + 3 * oe);
     if (s) sub3(dir, pown, poth); else sub3(dir, poth, pown);
@@ -656,27 +700,27 @@ TB_FN void smooth_dynamics(BarState<P>& B, EnvSh<P>& S, const ModelT<typename P:
     sub3(ro, poth, S.xpos + 3 * ob); cross3(cw, ro, dir);
     real voth = dot3(dir, S.vw + 6 * ob) + dot3(cw, S.vw + 6 * ob + 3);
     real vel = s ? (vown - voth) : (voth - vown);
-    real frc = 0, Bt = -m.tdamp[t];
-    if (m.tk[t] > 0) {
-      if (len > m.tls[t][1]) frc = m.tk[t] * (m.tls[t][1] - len);
-      else if (len < m.tls[t][0]) frc = m.tk[t] * (m.tls[t][0] - len);
+    real frc = 0, Bt = -prm_tdamp(R, m, t);
+    if (prm_tk(R, m, t) > 0) {
+      if (len > prm_tls(R, m, t, 1)) frc = prm_tk(R, m, t) * (prm_tls(R, m, t, 1) - len);
+      else if (len < prm_tls(R, m, t, 0)) frc = prm_tk(R, m, t) * (prm_tls(R, m, t, 0) - len);
     }
-    frc -= m.tdamp[t] * vel;
+    frc -= prm_tdamp(R, m, t) * vel;
     const int a = m.ten_act[t];
     if (a >= 0) {
       real ctrl = (real)S.ctrl[a], input;
       if (m.ctrllimited) ctrl = clampr(ctrl, m.ctrlrange[0], m.ctrlrange[1]);
       real act = (real)S.act[a];
-      if (m.dyntype) { if (s == 0) S.actdot[a] = (ctrl - act) / tmax(MINV, m.dynprm0); input = act; }
+      if (m.dyntype) { if (s == 0) S.actdot[a] = (ctrl - act) / tmax(MINV, prm_dynprm0(R, m)); input = act; }
       else { if (s == 0) S.actdot[a] = 0; input = ctrl; }
-      real fa = m.gain * input + m.bias[0] + m.bias[1] * len + m.bias[2] * vel;
+      real fa = prm_gain(R, m) * input + prm_bias(R, m, 0) + prm_bias(R, m, 1) * len + prm_bias(R, m, 2) * vel;
       bool clamped = false;
       if (m.forcelimited) {
         clamped = (fa <= m.forcerange[0] || fa >= m.forcerange[1]);
         fa = clampr(fa, m.forcerange[0], m.forcerange[1]);
       }
       frc += fa;
-      if (m.bias[2] != 0 && ((m.flags & 1u) || !clamped)) Bt += m.bias[2];
+      if (prm_bias(R, m, 2) != 0 && ((m.flags & 1u) || !clamped)) Bt += prm_bias(R, m, 2);
     }
     if (s == 0) S.tlen[t] = len;
     real sg = s ? frc : -frc;

@@ -47,6 +47,8 @@ struct StepIO {
   double* pool_real_obs;// [n_pool][obs_dim] or null: its noise-free twin (use_obs_noise)
   double* real_obs;     // [N][obs_dim] or null: noise-free observation when use_obs_noise (info["real_observation"])
   int* counter;         // work counter of the launch
+  double* params;       // per-env variant: [N + n_pool][NPARAM] parameter rows
+  const double* prange; // per-env variant: {nominal, lo, hi}[NPARAM] of the reset draws, or null = rows kept at resets
 };
 
 TB_FN double angle_normalize(double t) {  // tr_env.py:648-654
@@ -501,6 +503,31 @@ TB_FN void make_draws(double* d, unsigned long long seed, unsigned long long env
   }
 }
 
+// Per-env parameter row of a reset: row[i] = nominal[i] * U(lo[i], hi[i]), prange = {nominal, lo, hi}[NPARAM].  Draw j
+// of the 32 is u01 half j & 1 of Philox(seed ^ key, stream, (nreset << 8) | j / 2); the lower and upper spring length
+// of a tendon share one draw, so a deadband stays ordered.  The scale is rounded before the product (no fused
+// multiply-add) so that the host emulator draws the same rows bit for bit.
+TB_FN double draw_param(const double* prange, unsigned long long seed, unsigned long long stream, unsigned long long nreset, int i) {
+  const int j = i < PRM_TLS ? i : (i < PRM_GAIN ? PRM_TLS + (i - PRM_TLS) / 2 : i - NTEN);
+  uint32_t r[4];
+  philox(seed ^ 0x706172616d726e64ull, stream, (nreset << 8) | (unsigned long long)(j >> 1), r);
+  const double u = (j & 1) ? u01(r[2], r[3]) : u01(r[0], r[1]);
+  const double lo = prange[NPARAM + i], hi = prange[2 * NPARAM + i];
+#if TB_DEV
+  const double scale = __dadd_rn(lo, __dmul_rn(u, hi - lo));
+#else
+  const double scale = lo + u * (hi - lo);
+#endif
+  return prange[i] * scale;
+}
+TB_FN void draw_params(double* row, const double* prange, unsigned long long seed, unsigned long long stream, unsigned long long nreset) {
+  for (int i = 0; i < NPARAM; i++) row[i] = draw_param(prange, seed, stream, nreset, i);
+}
+// per-env variant: point the env's slice at its parameter row (lane 0; the caller's next wsync publishes it)
+template <typename PR> TB_FN void set_prm_row(EnvSh<PR>& S, const StepIO& io, size_t row) {
+  if constexpr (PR::per_env) S.prm = io.params + row * NPARAM;
+}
+
 constexpr int OBS_MAX = 160;
 
 // ---- the step of EPW consecutive envs starting at `first` (one warp)
@@ -511,7 +538,10 @@ TB_FN void run_step(EnvSh<PR>& S, const ModelT<typename PR::real>& m, const EnvC
   Aux A; StepOut O;
   double* rec = io.state + (size_t)(on ? e : 0) * STATE_STRIDE;
   load_env(S, L, on, A, rec, io.heading + (size_t)(on ? e : 0) * HEADING_SLOTS);
-  if (l0) for (int i = 0; i < NACT; i++) S.action[i] = io.ctrl64 ? io.ctrl64[(size_t)e * NACT + i] : (double)io.ctrl32[(size_t)e * NACT + i];
+  if (l0) {
+    for (int i = 0; i < NACT; i++) S.action[i] = io.ctrl64 ? io.ctrl64[(size_t)e * NACT + i] : (double)io.ctrl32[(size_t)e * NACT + i];
+    set_prm_row(S, io, (size_t)e);
+  }
   wsync();
   env_step(S, m, c, L, on, A, O, aligned);
   if (l0) {
@@ -560,6 +590,10 @@ TB_FN void run_reset(EnvSh<PR>& S, const ModelT<typename PR::real>& m, const Env
     if (!io.explicit_draws) make_draws(dr, io.seed, (unsigned long long)(io.env_id_base + e), (unsigned long long)nreset);
     A.draws = dr;
     A.nz_seed = io.seed; A.nz_stream = (unsigned long long)(io.env_id_base + e); A.nz_nreset = (unsigned long long)nreset;
+    if constexpr (PR::per_env) {
+      set_prm_row(S, io, (size_t)e);
+      if (io.prange) draw_params(io.params + (size_t)e * NPARAM, io.prange, io.seed, A.nz_stream, A.nz_nreset);
+    }
   }
   wsync();
   reset_begin(S, m, c, L, on, A);
@@ -601,6 +635,10 @@ TB_FN void run_pool(EnvSh<PR>& S, const ModelT<typename PR::real>& m, const EnvC
     if (phase == 0) make_draws(dr, io.seed, (1ull << 40) + (unsigned long long)(io.env_id_base + p), (unsigned long long)nreset);
     A.draws = dr;
     A.nz_seed = io.seed; A.nz_stream = (1ull << 40) + (unsigned long long)(io.env_id_base + p); A.nz_nreset = (unsigned long long)nreset;
+    if constexpr (PR::per_env) {   // the slot's row; tsg_assign hands it to the env together with the record
+      set_prm_row(S, io, row);
+      if (phase == 0 && io.prange) draw_params(io.params + row * NPARAM, io.prange, io.seed, A.nz_stream, A.nz_nreset);
+    }
   }
   wsync();
   const bool begin = on && phase == 0;
@@ -641,6 +679,10 @@ TB_FN void run_forward(EnvSh<PR>& S, const ModelT<typename PR::real>& m, const E
   Aux A;
   double* rec = io.state + (size_t)(on ? e : 0) * STATE_STRIDE;
   load_env(S, L, on, A, rec, io.heading + (size_t)(on ? e : 0) * HEADING_SLOTS);
+  if constexpr (PR::per_env) {
+    if (l0) set_prm_row(S, io, (size_t)e);
+    wsync();
+  }
   simulate(S, m, L, on, 1, false, false);
   if (l0) {
     aux_from_forward(S, A);

@@ -19,6 +19,9 @@ constexpr int INFO_DIM = 32;
 constexpr int HEADING_SLOTS = 32;
 constexpr int NDRAW = 10;
 constexpr double PI = 3.14159265358979323846;
+// per-env parameter row (include/tsg.h TSG_PARAM_*): absolute values in model units
+constexpr int NPARAM = 41;
+enum ParamOff { PRM_TK = 0, PRM_TDAMP = 9, PRM_TLS = 18 /* lower, upper per tendon */, PRM_GAIN = 36, PRM_BIAS = 37, PRM_DYNPRM0 = 40 };
 enum { ENV_TR = 0, ENV_LEGACY = 1 };
 enum { TASK_STRAIGHT = 0, TASK_TURN = 1, TASK_AIMING = 2, TASK_TRACKING = 3, TASK_VEL_TRACK = 4 };
 
@@ -173,6 +176,29 @@ inline std::string make_model(const TsgModel& t, ModelT<real>& m, const float* h
     m.hdata = hdata_dev;
     if (!hdata_dev || m.nrow < 2 || m.ncol < 2) return "height field data missing";
   }
+  return "";
+}
+
+// the nominal parameter row: the TsgModel fields make_model reads into tk / tdamp / tls / gain / bias / dynprm0
+inline void nominal_params(const TsgModel& t, double* row) {
+  for (int tt = 0; tt < NTEN; tt++) {
+    row[PRM_TK + tt] = t.ten_stiffness[tt]; row[PRM_TDAMP + tt] = t.ten_damping[tt];
+    row[PRM_TLS + 2 * tt] = t.ten_lengthspring[tt][0]; row[PRM_TLS + 2 * tt + 1] = t.ten_lengthspring[tt][1];
+  }
+  row[PRM_GAIN] = t.act_gain;
+  for (int k = 0; k < 3; k++) row[PRM_BIAS + k] = t.act_bias[k];
+  row[PRM_DYNPRM0] = t.act_dynprm0;
+}
+// scale ranges of the reset draws, lo / hi [NPARAM]; returns "" when valid
+inline std::string check_param_ranges(const double* lo, const double* hi) {
+  for (int i = 0; i < NPARAM; i++) {
+    if (!isfinite(lo[i]) || !isfinite(hi[i])) return "param ranges must be finite";
+    if (!(lo[i] >= 0 && lo[i] <= hi[i])) return "param ranges need 0 <= lo <= hi";
+  }
+  if (!(lo[PRM_DYNPRM0] > 0)) return "the act_dynprm0 scale must be above 0";
+  for (int tt = 0; tt < NTEN; tt++)
+    if (lo[PRM_TLS + 2 * tt] != lo[PRM_TLS + 2 * tt + 1] || hi[PRM_TLS + 2 * tt] != hi[PRM_TLS + 2 * tt + 1])
+      return "the lower and upper ten_lengthspring of a tendon share one draw: their ranges must be equal";
   return "";
 }
 

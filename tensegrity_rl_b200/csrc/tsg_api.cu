@@ -31,6 +31,9 @@ using namespace tb;
 static_assert(STATE_STRIDE == TSG_STATE_STRIDE && INFO_DIM == TSG_INFO_DIM && NDRAW == TSG_NDRAW, "ABI constants");
 static_assert(SO_USED <= STATE_STRIDE, "state record too small");
 static_assert(HEADING_SLOTS == TSG_HEADING_SLOTS, "heading slots");
+static_assert(NPARAM == TSG_NPARAM && PRM_TK == TSG_PARAM_TEN_STIFFNESS && PRM_TDAMP == TSG_PARAM_TEN_DAMPING &&
+              PRM_TLS == TSG_PARAM_TEN_LENGTHSPRING && PRM_GAIN == TSG_PARAM_ACT_GAIN && PRM_BIAS == TSG_PARAM_ACT_BIAS &&
+              PRM_DYNPRM0 == TSG_PARAM_ACT_DYNPRM0, "param row layout");
 
 enum { MODE_STEP = 0, MODE_RESET = 1, MODE_FORWARD = 2 };
 
@@ -168,6 +171,25 @@ __global__ void tsg_scatter_kernel(double* __restrict__ state, int n, const doub
   if (ctrl) for (int i = 0; i < NACT; i++) r[SO_CTRL + i] = ctrl[(size_t)e * NACT + i];
   if (act) for (int i = 0; i < NACT; i++) r[SO_ACT + i] = act[(size_t)e * NACT + i];
 }
+// per-env parameters: the k-th assigned pool slot's row goes to the k-th done env (the pairs tsg_assign_kernel chose)
+__global__ void tsg_assign_params_kernel(double* __restrict__ params, const int* __restrict__ lists, const int* __restrict__ counts,
+                                         int n, int n_pool) {
+  const int npair = counts[2];
+  for (int k = blockIdx.x; k < npair; k += gridDim.x) {
+    const int e = lists[k], p = lists[n_pool + k];
+    for (int i = threadIdx.x; i < NPARAM; i += blockDim.x) params[(size_t)e * NPARAM + i] = params[(size_t)(n + p) * NPARAM + i];
+  }
+}
+// rows [n][NPARAM] = nominal row
+__global__ void tsg_fill_params_kernel(double* __restrict__ rows, int n, const double* __restrict__ nominal) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < (size_t)n * NPARAM) rows[i] = nominal[i % NPARAM];
+}
+// rows of the envs whose mask byte is non-zero (mask NULL = all) = src rows
+__global__ void tsg_set_params_kernel(double* __restrict__ rows, int n, const double* __restrict__ src, const uint8_t* __restrict__ mask) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < (size_t)n * NPARAM && (!mask || mask[i / NPARAM])) rows[i] = src[i];
+}
 __global__ void tsg_init_records_kernel(double* __restrict__ state, int n, const double* qpos0) {  // n = envs + pool slots
   int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n) return;
@@ -190,14 +212,20 @@ struct TsgHandle {
   double* d_pool_obs; double* d_pool_real_obs; int* d_lists; int* d_counts; uint8_t* d_need_sync;
   double* real_obs;   // where the noise-free observation goes with use_obs_noise: d_realobs_own or the caller's buffer
   double* d_realobs_own;
+  // per-env parameters (off until tsg_set_param_ranges / tsg_set_env_params): rows [n_envs + n_pool][NPARAM] and
+  // {nominal, lo, hi}[NPARAM] of the reset draws
+  double* d_params; double* d_prange;
+  int per_env, ranges_on;
+  double nominal[NPARAM];
   int grid[3], grid_small, shape, regs, warps, epw;   // shape: 0 = TB_WARPS, 1 = TB_WARPS_SMALL warps per CTA in the step kernel
+  int pgrid[3], pgrid_small;   // grids of the per-env kernels
   size_t smem;
   cudaStream_t own_stream;
 };
 
 static thread_local std::string g_err;
 const char* tsg_last_error(void) { return g_err.c_str(); }
-int tsg_version(void) { return 2; }
+int tsg_version(void) { return 3; }
 int tsg_device_count(void) { int n = 0; if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; } return n; }
 
 #define CK(call)                                                                    \
@@ -227,13 +255,19 @@ static int launch_w(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot, 
 }
 template <typename P, int MODE>
 static int launch_t(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot) {
-  if (MODE == MODE_STEP && h->shape == 1) return launch_w<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, io, s, counter_slot, h->grid_small);
-  return launch_w<P, MODE, TB_WARPS>(h, io, s, counter_slot, h->grid[MODE]);
+  const int* grid = P::per_env ? h->pgrid : h->grid;
+  if (MODE == MODE_STEP && h->shape == 1) return launch_w<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, io, s, counter_slot, P::per_env ? h->pgrid_small : h->grid_small);
+  return launch_w<P, MODE, TB_WARPS>(h, io, s, counter_slot, grid[MODE]);
 }
 // counter_slot: which of the handle's work counters the launch consumes (they are zeroed together, once per API call)
 template <int MODE>
 static int launch_env(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot) {
-  return h->precision == TSG_PRECISION_F32 ? launch_t<P32, MODE>(h, io, s, counter_slot) : launch_t<P64, MODE>(h, io, s, counter_slot);
+  const bool f32 = h->precision == TSG_PRECISION_F32;
+  if (h->per_env) {
+    io.params = h->d_params; io.prange = h->ranges_on ? h->d_prange : nullptr;
+    return f32 ? launch_t<PerEnv<P32>, MODE>(h, io, s, counter_slot) : launch_t<PerEnv<P64>, MODE>(h, io, s, counter_slot);
+  }
+  return f32 ? launch_t<P32, MODE>(h, io, s, counter_slot) : launch_t<P64, MODE>(h, io, s, counter_slot);
 }
 static int zero_counters(TsgHandle* h, cudaStream_t s) {
   CK(cudaMemsetAsync(h->d_counter, 0, 4 * sizeof(int), s));
@@ -283,9 +317,18 @@ static int setup_model(TsgHandle* h, const TsgModel* model, int sms) {
       setup_kernel<P, MODE_RESET, TB_WARPS>(h, sms, &h->grid[MODE_RESET]) || setup_kernel<P, MODE_FORWARD, TB_WARPS>(h, sms, &h->grid[MODE_FORWARD])) return -2;
   h->shape = shape_override() >= 0 ? shape_override() : (small_one_wave ? 1 : 0);
   if (h->shape == 1 ? note_kernel<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<P, MODE_STEP, TB_WARPS>(h)) return -2;
-  int gmax = h->grid[0] > h->grid[1] ? h->grid[0] : h->grid[1];
-  if (h->grid[2] > gmax) gmax = h->grid[2];
-  size_t slots = (size_t)gmax * TB_WARPS > (size_t)h->grid_small * TB_WARPS_SMALL ? (size_t)gmax * TB_WARPS : (size_t)h->grid_small * TB_WARPS_SMALL;
+  // the per-env kernels (same CTA shapes, a wider env slice) share the contact spill area
+  typedef PerEnv<P> PE;
+  if (setup_kernel<PE, MODE_STEP, TB_WARPS>(h, sms, &h->pgrid[MODE_STEP]) ||
+      setup_kernel<PE, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, sms, &h->pgrid_small) ||
+      setup_kernel<PE, MODE_RESET, TB_WARPS>(h, sms, &h->pgrid[MODE_RESET]) || setup_kernel<PE, MODE_FORWARD, TB_WARPS>(h, sms, &h->pgrid[MODE_FORWARD])) return -2;
+  size_t slots = 0;
+  for (int k = 0; k < 3; k++) {
+    if ((size_t)h->grid[k] * TB_WARPS > slots) slots = (size_t)h->grid[k] * TB_WARPS;
+    if ((size_t)h->pgrid[k] * TB_WARPS > slots) slots = (size_t)h->pgrid[k] * TB_WARPS;
+  }
+  if ((size_t)h->grid_small * TB_WARPS_SMALL > slots) slots = (size_t)h->grid_small * TB_WARPS_SMALL;
+  if ((size_t)h->pgrid_small * TB_WARPS_SMALL > slots) slots = (size_t)h->pgrid_small * TB_WARPS_SMALL;
   CK(cudaMalloc(&h->d_spill, slots * EPW * (3 * KS) * sizeof(Con<typename P::sreal>)));   // contact slots beyond the shared-memory pool
   return 0;
 }
@@ -305,6 +348,7 @@ static int create_impl(TsgHandle* h, const TsgModel* model, const TsgEnvConfig* 
   std::string err = make_env_cfg(*cfg, *model, ec);
   if (!err.empty()) FAIL("tsg_create: " + err);
   h->obs_dim = ec.obs_dim; h->ready_phase = ec.warmup_steps + 1;
+  nominal_params(*model, h->nominal);
   size_t n = (size_t)n_envs + (size_t)n_pool;
   CK(cudaMalloc(&h->d_cfg, sizeof(EnvCfg)));
   CK(cudaMemcpy(h->d_cfg, &ec, sizeof(ec), cudaMemcpyHostToDevice));
@@ -373,7 +417,7 @@ int tsg_destroy(TsgHandle* h) {
   cudaSetDevice(h->device);
   void* ptrs[] = {h->d_model, h->d_cfg, h->d_hdata, h->d_qpos0, h->d_state, h->d_heading, h->d_draws, h->d_done, h->d_ctrl,
                   h->d_obs, h->d_reward, h->d_info, h->d_termobs, h->d_tmp, h->d_mask, h->d_counter, h->d_spill, h->d_pool_obs,
-                  h->d_pool_real_obs, h->d_lists, h->d_counts, h->d_need_sync, h->d_realobs_own};
+                  h->d_pool_real_obs, h->d_lists, h->d_counts, h->d_need_sync, h->d_realobs_own, h->d_params, h->d_prange};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   delete h;
@@ -450,6 +494,11 @@ int tsg_step(TsgHandle* h, const void* ctrl_dev, int ctrl_dtype, double* obs_dev
                                            h->n_pool, h->obs_dim, h->ready_phase);
       CK(cudaGetLastError());
       h->launches++;
+      if (h->per_env) {
+        tsg_assign_params_kernel<<<h->n_pool < 1024 ? h->n_pool : 1024, 64, 0, s>>>(h->d_params, h->d_lists, h->d_counts, h->n_envs, h->n_pool);
+        CK(cudaGetLastError());
+        h->launches++;
+      }
       mask = h->d_need_sync;
     }
     StepIO r = base_io(h);
@@ -481,6 +530,82 @@ int tsg_forward(TsgHandle* h, double* obs_dev, double* info_dev, void* stream) {
   io.obs = obs_dev; io.info = info_dev;
   if (zero_counters(h, (cudaStream_t)stream)) return -2;
   return launch_env<MODE_FORWARD>(h, io, (cudaStream_t)stream, 0);
+}
+
+// ---- per-env parameters
+// first use: rows of every env and pool slot = the nominal row, and the handle switches to the per-env kernels
+static int enable_params(TsgHandle* h) {
+  if (h->per_env) return 0;
+  size_t n = (size_t)h->n_envs + (size_t)h->n_pool;
+  double pr[3 * NPARAM];
+  for (int i = 0; i < NPARAM; i++) { pr[i] = h->nominal[i]; pr[NPARAM + i] = 1; pr[2 * NPARAM + i] = 1; }
+  if (!h->d_prange) CK(cudaMalloc(&h->d_prange, sizeof(pr)));
+  CK(cudaMalloc(&h->d_params, n * NPARAM * sizeof(double)));
+  CK(cudaDeviceSynchronize());
+  CK(cudaMemcpy(h->d_prange, pr, sizeof(pr), cudaMemcpyHostToDevice));
+  tsg_fill_params_kernel<<<(int)((n * NPARAM + 255) / 256), 256>>>(h->d_params, (int)n, h->d_prange);
+  CK(cudaGetLastError());
+  CK(cudaDeviceSynchronize());
+  int rc;
+  if (h->precision == TSG_PRECISION_F32) rc = h->shape == 1 ? note_kernel<PerEnv<P32>, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<PerEnv<P32>, MODE_STEP, TB_WARPS>(h);
+  else rc = h->shape == 1 ? note_kernel<PerEnv<P64>, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<PerEnv<P64>, MODE_STEP, TB_WARPS>(h);
+  if (rc) return rc;
+  h->per_env = 1;
+  return 0;
+}
+
+int tsg_set_param_ranges(TsgHandle* h, const double* lo, const double* hi) {
+  if (!h) FAIL("tsg_set_param_ranges: null handle");
+  if (!lo != !hi) FAIL("tsg_set_param_ranges: lo and hi must both be given or both be NULL");
+  CK(cudaSetDevice(h->device));
+  if (!lo) {   // off: rows stay as they are at later resets
+    if (h->per_env) { CK(cudaDeviceSynchronize()); h->ranges_on = 0; }
+    return 0;
+  }
+  std::string err = check_param_ranges(lo, hi);
+  if (!err.empty()) FAIL("tsg_set_param_ranges: " + err);
+  int rc = enable_params(h);
+  if (rc) return rc;
+  CK(cudaDeviceSynchronize());   // no launch in flight reads the ranges being replaced
+  CK(cudaMemcpy(h->d_prange + NPARAM, lo, NPARAM * sizeof(double), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(h->d_prange + 2 * NPARAM, hi, NPARAM * sizeof(double), cudaMemcpyHostToDevice));
+  h->ranges_on = 1;
+  return 0;
+}
+
+int tsg_set_env_params(TsgHandle* h, const double* params_dev, const uint8_t* mask_dev, void* stream) {
+  if (!h || !params_dev) FAIL("tsg_set_env_params: null argument");
+  if (h->n_pool > 0)
+    FAIL("tsg_set_env_params: the handle has a reset pool; an env that receives a pool slot takes the slot's row, "
+         "which would replace an explicit row (create the handle with n_pool = 0)");
+  CK(cudaSetDevice(h->device));
+  int rc = enable_params(h);
+  if (rc) return rc;
+  size_t cnt = (size_t)h->n_envs * NPARAM;
+  tsg_set_params_kernel<<<(int)((cnt + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_params, h->n_envs, params_dev, mask_dev);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int tsg_get_env_params(TsgHandle* h, double* params_dev, void* stream) {
+  if (!h || !params_dev) FAIL("tsg_get_env_params: null argument");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  size_t cnt = (size_t)h->n_envs * NPARAM;
+  if (h->per_env) {
+    CK(cudaMemcpyAsync(params_dev, h->d_params, cnt * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    return 0;
+  }
+  // without per-env parameters every env runs the nominal row; the nominal row comes from the host once
+  if (!h->d_prange) {
+    CK(cudaMalloc(&h->d_prange, 3 * NPARAM * sizeof(double)));
+    CK(cudaMemcpy(h->d_prange, h->nominal, NPARAM * sizeof(double), cudaMemcpyHostToDevice));
+  }
+  tsg_fill_params_kernel<<<(int)((cnt + 255) / 256), 256, 0, s>>>(params_dev, h->n_envs, h->d_prange);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
 }
 
 // ---- host-buffer helpers

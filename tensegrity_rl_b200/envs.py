@@ -58,7 +58,9 @@ class _SingleEnv:
     metadata = {"render_modes": ["human", "rgb_array", "depth_array"], "render_fps": 50}
 
     def __init__(self, xml_file=os.path.join(os.getcwd(), "3prism_jonathan_steady_side.xml"), device=0, seed=0,
-                 max_episode_steps=0, render_mode=None, **kwargs):
+                 max_episode_steps=0, render_mode=None, param_ranges=None, **kwargs):
+        """param_ranges: per-env tendon and actuator parameters redrawn at every reset, {field: (lo, hi)} scale
+        factors (TensegrityVecEnv.set_param_ranges)"""
         self.L = _lib.load()
         for k in ("width", "height", "camera_id", "camera_name", "contact_with_self_penalty",
                   "use_cap_size_noise", "cap_size_noise_range", "threshold_waypt"):
@@ -76,6 +78,9 @@ class _SingleEnv:
         h = C.c_void_p()
         _lib.check(self.L.tsg_create(C.byref(self._model), C.byref(self.cfg), 1, int(device), 0, C.byref(h)))
         self.h = h
+        if param_ranges is not None:
+            lo, hi = M.param_scale_ranges(param_ranges)
+            _lib.check(self.L.tsg_set_param_ranges(self.h, self._p(lo), self._p(hi)))
         lo, hi = self.md["ctrlrange"]
         self.action_space = Box(np.full(6, lo, np.float32), np.full(6, hi, np.float32), dtype=np.float32)
         # use_contact_forces: the reference DECLARES 84 more observation slots (tr_env.py:263-264) but its _get_obs never

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 
 from . import build as _build
+from . import model as _M
 from .model import TsgEnvConfig, TsgModel
 
 STATE_STRIDE, INFO_DIM, NDRAW, HEADING_SLOTS = 96, 32, 10, 32
@@ -11,12 +12,16 @@ CTRL_F64, CTRL_F32 = 0, 1
 INFO = dict(rew_fwd=0, rew_ctrl=1, rew_survive=2, x=3, y=4, psi=5, xvel=6, yvel=7, ten=8, terminated=17,
             truncated=18, ncon=19, niter=20, nls=21, barforce=22, maxcfrc=23, waypt=24, ori=26, overflow=28,
             bad=29, nmpr=30, reset_psi=31)
+# per-env parameter row (TSG_PARAM_*): field -> slice of the TSG_NPARAM doubles
+NPARAM = _M.NPARAM
+PARAM = {name: slice(off, off + w) for name, off, w in _M.PARAM_FIELDS}
 
 SYMBOLS = ["tsg_last_error", "tsg_version", "tsg_device_count", "tsg_create", "tsg_create_pooled", "tsg_pool_stats_host", "tsg_destroy", "tsg_num_envs",
            "tsg_obs_dim", "tsg_launches", "tsg_kernel_config", "tsg_reset", "tsg_step", "tsg_forward",
            "tsg_get_state_host", "tsg_set_state_host", "tsg_get_records_host", "tsg_set_records_host",
            "tsg_get_draws_host", "tsg_step_host", "tsg_reset_host", "tsg_set_real_obs", "tsg_get_real_obs_host",
-           "tsg_create_opts", "tsg_precision", "tsg_forward_host", "tsg_get_heading_host", "tsg_set_heading_host"]
+           "tsg_create_opts", "tsg_precision", "tsg_forward_host", "tsg_get_heading_host", "tsg_set_heading_host",
+           "tsg_set_param_ranges", "tsg_set_env_params", "tsg_get_env_params"]
 PRECISION = {"f64": 0, "f32": 1}
 
 
@@ -64,6 +69,9 @@ def load():
     L.tsg_reset_host.argtypes = [vp, u8p, C.c_ulonglong, dp, dp]
     L.tsg_set_real_obs.argtypes = [vp, dp]
     L.tsg_get_real_obs_host.argtypes = [vp, dp]
+    L.tsg_set_param_ranges.argtypes = [vp, dp, dp]
+    L.tsg_set_env_params.argtypes = [vp, dp, u8p, vp]
+    L.tsg_get_env_params.argtypes = [vp, dp, vp]
     _lib = L
     return L
 

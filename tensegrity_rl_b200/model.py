@@ -365,6 +365,71 @@ def model_struct(md):
     return m, keep
 
 
+# --------------------------------------------------------------------------- per-env parameters
+# the row layout of include/tsg.h (TSG_PARAM_*): field -> (offset, width)
+PARAM_FIELDS = (("ten_stiffness", 0, NTEN), ("ten_damping", 9, NTEN), ("ten_lengthspring", 18, 2 * NTEN),
+                ("act_gain", 36, 1), ("act_bias", 37, 3), ("act_dynprm0", 40, 1))
+NPARAM = 41
+
+
+def nominal_params(md):
+    """the nominal per-env parameter row [41] of a model dict: its tendon and actuator constants"""
+    row = np.zeros(NPARAM)
+    for name, off, w in PARAM_FIELDS:
+        row[off:off + w] = np.asarray(md[name], np.float64).reshape(-1)
+    return row
+
+
+def param_overrides(row):
+    """per-env parameter row [41] -> the model-dict fields it replaces (keyword overrides of a model dict)"""
+    row = np.asarray(row, np.float64)
+    if row.shape != (NPARAM,):
+        raise ValueError(f"a parameter row has {NPARAM} values, got shape {row.shape}")
+    out = {}
+    for name, off, w in PARAM_FIELDS:
+        v = row[off:off + w]
+        if name == "ten_lengthspring":
+            out[name] = v.reshape(NTEN, 2).tolist()
+        elif w == 1:
+            out[name] = float(v[0])
+        else:
+            out[name] = v.tolist()
+    return out
+
+
+def param_scale_ranges(param_ranges):
+    """{field: (lo, hi)} of scale factors (each bound a scalar or an array of the field's width; fields not given
+    keep scale 1) -> (lo[41], hi[41]).  Raises ValueError on an unknown field, a bad shape, a non-finite bound,
+    lo > hi, a negative scale, a dynprm0 scale of 0, or unequal ranges of a tendon's lower and upper lengthspring."""
+    lo, hi = np.ones(NPARAM), np.ones(NPARAM)
+    fields = {name: (off, w) for name, off, w in PARAM_FIELDS}
+    for name, bounds in dict(param_ranges).items():
+        if name not in fields:
+            raise ValueError(f"unknown per-env parameter {name!r}; known: {', '.join(fields)}")
+        off, w = fields[name]
+        try:
+            b_lo, b_hi = bounds
+        except (TypeError, ValueError):
+            raise ValueError(f"{name}: expected a (lo, hi) pair") from None
+        for dst, b in ((lo, b_lo), (hi, b_hi)):
+            a = np.asarray(b, np.float64)
+            if a.ndim == 0:
+                a = np.full(w, float(a))
+            if a.shape != (w,):
+                raise ValueError(f"{name}: a bound is a scalar or has {w} values, got shape {a.shape}")
+            dst[off:off + w] = a
+    if not (np.isfinite(lo).all() and np.isfinite(hi).all()):
+        raise ValueError("param ranges must be finite")
+    if (lo < 0).any() or (lo > hi).any():
+        raise ValueError("param ranges need 0 <= lo <= hi")
+    if not lo[40] > 0:
+        raise ValueError("the act_dynprm0 scale must be above 0")
+    ls = slice(18, 36)
+    if not (np.array_equal(lo[ls][0::2], lo[ls][1::2]) and np.array_equal(hi[ls][0::2], hi[ls][1::2])):
+        raise ValueError("the lower and upper ten_lengthspring of a tendon share one draw: their ranges must be equal")
+    return lo, hi
+
+
 # --------------------------------------------------------------------------- env config
 def load_reset_poses():
     with open(os.path.join(ASSET_DIR, "reset_poses.json")) as f:

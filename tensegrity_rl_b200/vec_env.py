@@ -26,11 +26,15 @@ class TensegrityVecEnv:
     metadata = {"render_modes": []}
 
     def __init__(self, num_envs, xml_file=None, env="tr_env", device=0, seed=0, env_id_base=0,
-                 auto_reset=True, info_mode="auto", max_episode_steps=5000, reset_pool=0, precision="f64", **env_kwargs):
+                 auto_reset=True, info_mode="auto", max_episode_steps=5000, reset_pool=0, precision="f64",
+                 param_ranges=None, **env_kwargs):
         """reset_pool: number of background reset slots (0 = every reset runs synchronously, bit-reproducible per
         env id; "auto" = num_envs // 4, at least 32).  With a pool, an env that is done receives a slot that has
         already been through the reference's 50-step reset warm-up, so resets add no latency to a step.
-        precision: "f64" (the reference's arithmetic, default) or "f32" (optional fp32 physics)."""
+        precision: "f64" (the reference's arithmetic, default) or "f32" (optional fp32 physics).
+        param_ranges: per-env tendon and actuator parameters redrawn at every reset (domain randomisation), as
+        {field: (lo, hi)} scale factors of the nominal value; fields are those of `lib.PARAM`, each bound a scalar or an
+        array of the field's width, fields not given keep scale 1.  See set_param_ranges."""
         import torch
 
         if not torch.cuda.is_available():
@@ -76,6 +80,8 @@ class TensegrityVecEnv:
                 _lib.check(self.L.tsg_set_real_obs(self.h, _ptr(self.real_obs)))
         self._actions = None
         self.n_steps = 0
+        if param_ranges is not None:
+            self.set_param_ranges(param_ranges)
 
     # ------------------------------------------------------------------ torch (device) path
     def _stream(self):
@@ -116,6 +122,40 @@ class TensegrityVecEnv:
         with self.torch.cuda.device(self.device):
             _lib.check(self.L.tsg_forward(self.h, _ptr(self.obs), _ptr(self.info), self._stream()))
         return self.obs
+
+    # ------------------------------------------------------------------ per-env parameters
+    def set_param_ranges(self, param_ranges):
+        """From now on every reset draws each env's parameter row as nominal * U(lo, hi) per field (the lower and upper
+        ten_lengthspring of a tendon share one draw).  None stops the draws; rows then stay as they are.  The first
+        call switches the handle to the per-env kernels."""
+        if param_ranges is None:
+            _lib.check(self.L.tsg_set_param_ranges(self.h, None, None))
+            return
+        lo, hi = M.param_scale_ranges(param_ranges)
+        _lib.check(self.L.tsg_set_param_ranges(self.h, C.c_void_p(lo.ctypes.data), C.c_void_p(hi.ctypes.data)))
+
+    def set_env_params(self, params, mask=None):
+        """explicit parameter rows [N, 41] (absolute values, layout `lib.PARAM`) for all envs or those with mask != 0,
+        from the next step on; with param_ranges set they last until the env's next reset.  Not on a handle with a
+        reset pool (an env that receives a pool slot takes the slot's row)."""
+        t = self.torch
+        params = t.as_tensor(params, dtype=t.float64, device=self.device).contiguous()
+        if params.shape != (self.num_envs, _lib.NPARAM):
+            raise ValueError(f"params must have shape ({self.num_envs}, {_lib.NPARAM}), got {tuple(params.shape)}")
+        if mask is not None:
+            mask = t.as_tensor(mask, device=self.device).to(t.uint8).contiguous()
+        with t.cuda.device(self.device):
+            _lib.check(self.L.tsg_set_env_params(self.h, _ptr(params), _ptr(mask), self._stream()))
+            if params.device.type == "cuda":   # the copy is stream ordered: keep the source alive until it ran
+                params.record_stream(t.cuda.current_stream(self.device))
+
+    def get_env_params(self):
+        """every env's parameter row, a cuda float64 tensor [N, 41] (the nominal row until per-env parameters are on)"""
+        t = self.torch
+        out = t.empty(self.num_envs, _lib.NPARAM, dtype=t.float64, device=self.device)
+        with t.cuda.device(self.device):
+            _lib.check(self.L.tsg_get_env_params(self.h, _ptr(out), self._stream()))
+        return out
 
     # ------------------------------------------------------------------ SB3 VecEnv protocol (host numpy)
     def reset(self):
