@@ -3,6 +3,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -24,9 +25,6 @@ using namespace tb;
 #ifndef TB_WARPS_SMALL
 #define TB_WARPS_SMALL 2   // second CTA shape of the step kernel (two CTAs per SM), for batches that fit the machine at once
 #endif
-#ifndef TB_EPW_SMALL
-#define TB_EPW_SMALL 10    // envs per warp in that shape (fewer envs per warp = fewer envs waiting for the slowest one)
-#endif
 
 static_assert(STATE_STRIDE == TSG_STATE_STRIDE && INFO_DIM == TSG_INFO_DIM && NDRAW == TSG_NDRAW, "ABI constants");
 static_assert(SO_USED <= STATE_STRIDE, "state record too small");
@@ -42,14 +40,14 @@ template <typename P> __host__ __device__ constexpr size_t smem_model() { return
 constexpr size_t SMEM_CFG = align16(sizeof(EnvCfg));
 // env slices are spaced by an odd number of 16-byte units, so that the same field of the ten envs of a warp falls into different banks
 template <typename P> __host__ __device__ constexpr size_t envsh_stride() { return align16(sizeof(EnvSh<P>)) | 16; }
-template <typename P, int W, int E = EPW> constexpr size_t smem_bytes() { return smem_model<P>() + SMEM_CFG + (size_t)W * E * envsh_stride<P>(); }
+template <typename P, int W> constexpr size_t smem_bytes() { return smem_model<P>() + SMEM_CFG + (size_t)W * EPW * envsh_stride<P>(); }
 
 // Persistent CTAs: the grid fills the machine once (SMs x resident CTAs) and every CTA pulls rounds of TB_WARPS chunks
 // (a chunk = EPW consecutive envs, or pool slots, stepped by one warp) from a global counter until the batch is done,
 // so rounds of different cost (contact count, Newton iterations, resets) balance dynamically.  The env rounds come
 // first, then the pool rounds, so that all warps of a CTA always run the same program.  The model constants are
 // staged once per CTA in shared memory.
-template <typename P, int MODE, int W, int E = EPW>
+template <typename P, int MODE, int W>
 __global__ void __launch_bounds__(W * 32, TB_MIN_CTAS) tb_env_kernel(const ModelT<typename P::real>* __restrict__ gm,
                                                                             const EnvCfg* __restrict__ gc, StepIO io,
                                                                             Con<typename P::sreal>* __restrict__ spill_base) {
@@ -67,14 +65,14 @@ __global__ void __launch_bounds__(W * 32, TB_MIN_CTAS) tb_env_kernel(const Model
   __syncthreads();
   const ModelT<real>& m = *reinterpret_cast<const ModelT<real>*>(tb_smem);
   const EnvCfg& c = *reinterpret_cast<const EnvCfg*>(tb_smem + smem_model<P>());
-  const LaneCtx L = make_lane(E);
+  const LaneCtx L = make_lane();
   const int warp = threadIdx.x >> 5;
   EnvSh<P>& S = *reinterpret_cast<EnvSh<P>*>(tb_smem + smem_model<P>() + SMEM_CFG +
-                                                   (size_t)(warp * E + L.grp) * envsh_stride<P>());
+                                                   (size_t)(warp * EPW + L.grp) * envsh_stride<P>());
   if (L.valid && L.bar == 0) S.spill = spill_base + (size_t)((blockIdx.x * W + warp) * EPW + L.grp) * (3 * KS);
   __syncwarp();
-  const int env_chunks = (io.n_envs + E - 1) / E, env_rounds = (env_chunks + W - 1) / W;
-  const int pool_chunks = (MODE == MODE_STEP || (MODE == MODE_RESET && !io.mask)) ? (io.n_pool + E - 1) / E : 0;
+  const int env_chunks = (io.n_envs + EPW - 1) / EPW, env_rounds = (env_chunks + W - 1) / W;
+  const int pool_chunks = (MODE == MODE_STEP || (MODE == MODE_RESET && !io.mask)) ? (io.n_pool + EPW - 1) / EPW : 0;
   const int pool_rounds = (pool_chunks + W - 1) / W;
   for (;;) {
     __syncthreads();
@@ -83,11 +81,11 @@ __global__ void __launch_bounds__(W * 32, TB_MIN_CTAS) tb_env_kernel(const Model
     const int round = s_round;
     if (round >= env_rounds + pool_rounds) break;
     if (round < env_rounds) {
-      const int first = (round * W + warp) * E;   // may lie beyond the batch: the warp then idles in step
+      const int first = (round * W + warp) * EPW;   // may lie beyond the batch: the warp then idles in step
       if (MODE == MODE_STEP) run_step(S, m, c, io, L, first, true);
       else if (MODE == MODE_RESET) run_reset(S, m, c, io, L, first);
       else run_forward(S, m, c, io, L, first);
-    } else run_pool(S, m, c, io, L, ((round - env_rounds) * W + warp) * E, MODE == MODE_RESET);
+    } else run_pool(S, m, c, io, L, ((round - env_rounds) * W + warp) * EPW, MODE == MODE_RESET);
   }
 }
 
@@ -199,6 +197,7 @@ __global__ void tsg_init_records_kernel(double* __restrict__ state, int n, const
 }
 
 // ------------------------------------------------------------------ handle
+enum { STEP_SMALL = 3 };   // grid slot of the step kernel in the TB_WARPS_SMALL shape, after the TB_WARPS slots of the modes
 struct TsgHandle {
   int device, n_envs, n_pool, obs_dim, launches, ready_phase, precision;
   long long env_id_base;
@@ -217,8 +216,8 @@ struct TsgHandle {
   double* d_params; double* d_prange;
   int per_env, ranges_on;
   double nominal[NPARAM];
-  int grid[3], grid_small, shape, regs, warps, epw;   // shape: 0 = TB_WARPS, 1 = TB_WARPS_SMALL warps per CTA in the step kernel
-  int pgrid[3], pgrid_small;   // grids of the per-env kernels
+  int grid[2][4];           // [variant: default, per-env][MODE_STEP, MODE_RESET, MODE_FORWARD, STEP_SMALL]
+  int shape, regs;        // shape: 0 = TB_WARPS, 1 = TB_WARPS_SMALL warps per CTA in the step kernel
   size_t smem;
   cudaStream_t own_stream;
 };
@@ -244,10 +243,10 @@ static size_t extra_smem() {
   if (v < 0) { const char* e = getenv("TSG_EXTRA_SMEM"); v = e ? atol(e) : 0; }
   return (size_t)v;
 }
-template <typename P, int MODE, int W, int E = EPW>
+template <typename P, int MODE, int W>
 static int launch_w(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot, int grid) {
   io.counter = h->d_counter + counter_slot;
-  tb_env_kernel<P, MODE, W, E><<<grid, W * 32, smem_bytes<P, W, E>() + extra_smem(), s>>>(
+  tb_env_kernel<P, MODE, W><<<grid, W * 32, smem_bytes<P, W>() + extra_smem(), s>>>(
       (const ModelT<typename P::real>*)h->d_model, h->d_cfg, io, (Con<typename P::sreal>*)h->d_spill);
   CK(cudaGetLastError());
   h->launches++;
@@ -255,8 +254,8 @@ static int launch_w(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot, 
 }
 template <typename P, int MODE>
 static int launch_t(TsgHandle* h, StepIO& io, cudaStream_t s, int counter_slot) {
-  const int* grid = P::per_env ? h->pgrid : h->grid;
-  if (MODE == MODE_STEP && h->shape == 1) return launch_w<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, io, s, counter_slot, P::per_env ? h->pgrid_small : h->grid_small);
+  const int* grid = h->grid[P::per_env];
+  if (MODE == MODE_STEP && h->shape == 1) return launch_w<P, MODE_STEP, TB_WARPS_SMALL>(h, io, s, counter_slot, grid[STEP_SMALL]);
   return launch_w<P, MODE, TB_WARPS>(h, io, s, counter_slot, grid[MODE]);
 }
 // counter_slot: which of the handle's work counters the launch consumes (they are zeroed together, once per API call)
@@ -273,33 +272,44 @@ static int zero_counters(TsgHandle* h, cudaStream_t s) {
   CK(cudaMemsetAsync(h->d_counter, 0, 4 * sizeof(int), s));
   return 0;
 }
-template <typename P, int MODE, int W, int E = EPW>
+template <typename P, int MODE, int W>
 static int setup_kernel(TsgHandle* h, int num_sms, int* grid, bool* one_wave = nullptr) {
-  size_t smem = smem_bytes<P, W, E>() + extra_smem();
-  CK(cudaFuncSetAttribute(tb_env_kernel<P, MODE, W, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  size_t smem = smem_bytes<P, W>() + extra_smem();
+  CK(cudaFuncSetAttribute(tb_env_kernel<P, MODE, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tb_env_kernel<P, MODE, W, E>, W * 32, smem));
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tb_env_kernel<P, MODE, W>, W * 32, smem));
   if (per_sm < 1) { g_err = "tsg_create: kernel does not fit on an SM"; return -1; }
   // what is not carved out for shared memory stays L1, which serves the spilled contacts and the lanes' local memory
-  int need = ((h->n_envs + E - 1) / E + W - 1) / W + ((h->n_pool + E - 1) / E + W - 1) / W;
+  int need = ((h->n_envs + EPW - 1) / EPW + W - 1) / W + ((h->n_pool + EPW - 1) / EPW + W - 1) / W;
   int full = num_sms * per_sm;
   *grid = need < full ? need : full;
   if (one_wave) *one_wave = need <= full;
   return 0;
 }
-template <typename P, int MODE, int W, int E = EPW>
-static int note_kernel(TsgHandle* h) {
+// one row of the handle's grid table; small_one_wave: whether the small step shape covers the batch in one wave
+template <typename P>
+static int setup_variant(TsgHandle* h, int sms, bool* small_one_wave) {
+  int* grid = h->grid[P::per_env];
+  if (setup_kernel<P, MODE_STEP, TB_WARPS>(h, sms, &grid[MODE_STEP]) ||
+      setup_kernel<P, MODE_STEP, TB_WARPS_SMALL>(h, sms, &grid[STEP_SMALL], small_one_wave) ||
+      setup_kernel<P, MODE_RESET, TB_WARPS>(h, sms, &grid[MODE_RESET]) || setup_kernel<P, MODE_FORWARD, TB_WARPS>(h, sms, &grid[MODE_FORWARD])) return -2;
+  return 0;
+}
+// what tsg_kernel_config reports: the step kernel of variant and precision P in the handle's CTA shape
+template <typename P>
+static int note_step_kernel(TsgHandle* h) {
+  const bool small = h->shape == 1;
   cudaFuncAttributes a;
-  CK(cudaFuncGetAttributes(&a, tb_env_kernel<P, MODE, W, E>));
-  h->regs = a.numRegs; h->smem = smem_bytes<P, W, E>() + extra_smem(); h->warps = W; h->epw = E;
+  CK(cudaFuncGetAttributes(&a, small ? tb_env_kernel<P, MODE_STEP, TB_WARPS_SMALL> : tb_env_kernel<P, MODE_STEP, TB_WARPS>));
+  h->regs = a.numRegs; h->smem = (small ? smem_bytes<P, TB_WARPS_SMALL>() : smem_bytes<P, TB_WARPS>()) + extra_smem();
   return 0;
 }
 // CTA shape of the step kernel.  A batch that fits the machine at once in the small shape (2 CTAs of TB_WARPS_SMALL
 // warps per SM) is latency bound by a single round, which is shorter with fewer envs waiting for the slowest one at
 // the alignment barriers (4096 envs, steady state: 815k env-steps/s against 740k); larger batches run many rounds per
-// SM and the wide shape has the better throughput (131 072 envs: 1.40M against 1.20M).  Fewer envs per warp in the
-// small shape (TB_EPW_SMALL 5 or 4 with 3-4 warps) shorten a round only when the machine has room: +8 % at 2048 envs,
-// -7 to -14 % at 4096 (more warps per SM, each slower), so the default stays 10.  profiles/r2_ab_variants.log.
+// SM and the wide shape has the better throughput (131 072 envs: 1.40M against 1.20M).  Both shapes keep ten envs per
+// warp: 5 or 4 envs per warp with 3-4 warps in the small shape shortened a round only when the machine had room (+8 %
+// at 2048 envs) and lost 7 to 14 % at 4096 (more warps per SM, each slower).  profiles/r2_ab_variants.log.
 static int shape_override() {
   const char* e = getenv("TSG_SHAPE");
   return (e && (e[0] == '0' || e[0] == '1')) ? e[0] - '0' : -1;
@@ -312,23 +322,13 @@ static int setup_model(TsgHandle* h, const TsgModel* model, int sms) {
   CK(cudaMalloc(&h->d_model, sizeof(dm)));
   CK(cudaMemcpy(h->d_model, &dm, sizeof(dm), cudaMemcpyHostToDevice));
   bool small_one_wave = false;
-  if (setup_kernel<P, MODE_STEP, TB_WARPS>(h, sms, &h->grid[MODE_STEP]) ||
-      setup_kernel<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, sms, &h->grid_small, &small_one_wave) ||
-      setup_kernel<P, MODE_RESET, TB_WARPS>(h, sms, &h->grid[MODE_RESET]) || setup_kernel<P, MODE_FORWARD, TB_WARPS>(h, sms, &h->grid[MODE_FORWARD])) return -2;
+  if (setup_variant<P>(h, sms, &small_one_wave) || setup_variant<PerEnv<P>>(h, sms, nullptr)) return -2;
   h->shape = shape_override() >= 0 ? shape_override() : (small_one_wave ? 1 : 0);
-  if (h->shape == 1 ? note_kernel<P, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<P, MODE_STEP, TB_WARPS>(h)) return -2;
-  // the per-env kernels (same CTA shapes, a wider env slice) share the contact spill area
-  typedef PerEnv<P> PE;
-  if (setup_kernel<PE, MODE_STEP, TB_WARPS>(h, sms, &h->pgrid[MODE_STEP]) ||
-      setup_kernel<PE, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h, sms, &h->pgrid_small) ||
-      setup_kernel<PE, MODE_RESET, TB_WARPS>(h, sms, &h->pgrid[MODE_RESET]) || setup_kernel<PE, MODE_FORWARD, TB_WARPS>(h, sms, &h->pgrid[MODE_FORWARD])) return -2;
+  if (note_step_kernel<P>(h)) return -2;
+  // both variants share the contact spill area: EPW envs' slots for every warp of the largest launch
   size_t slots = 0;
-  for (int k = 0; k < 3; k++) {
-    if ((size_t)h->grid[k] * TB_WARPS > slots) slots = (size_t)h->grid[k] * TB_WARPS;
-    if ((size_t)h->pgrid[k] * TB_WARPS > slots) slots = (size_t)h->pgrid[k] * TB_WARPS;
-  }
-  if ((size_t)h->grid_small * TB_WARPS_SMALL > slots) slots = (size_t)h->grid_small * TB_WARPS_SMALL;
-  if ((size_t)h->pgrid_small * TB_WARPS_SMALL > slots) slots = (size_t)h->pgrid_small * TB_WARPS_SMALL;
+  for (int v = 0; v < 2; v++)
+    for (int k = 0; k < 4; k++) slots = std::max(slots, (size_t)h->grid[v][k] * (k == STEP_SMALL ? TB_WARPS_SMALL : TB_WARPS));
   CK(cudaMalloc(&h->d_spill, slots * EPW * (3 * KS) * sizeof(Con<typename P::sreal>)));   // contact slots beyond the shared-memory pool
   return 0;
 }
@@ -546,9 +546,7 @@ static int enable_params(TsgHandle* h) {
   tsg_fill_params_kernel<<<(int)((n * NPARAM + 255) / 256), 256>>>(h->d_params, (int)n, h->d_prange);
   CK(cudaGetLastError());
   CK(cudaDeviceSynchronize());
-  int rc;
-  if (h->precision == TSG_PRECISION_F32) rc = h->shape == 1 ? note_kernel<PerEnv<P32>, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<PerEnv<P32>, MODE_STEP, TB_WARPS>(h);
-  else rc = h->shape == 1 ? note_kernel<PerEnv<P64>, MODE_STEP, TB_WARPS_SMALL, TB_EPW_SMALL>(h) : note_kernel<PerEnv<P64>, MODE_STEP, TB_WARPS>(h);
+  int rc = h->precision == TSG_PRECISION_F32 ? note_step_kernel<PerEnv<P32>>(h) : note_step_kernel<PerEnv<P64>>(h);
   if (rc) return rc;
   h->per_env = 1;
   return 0;

@@ -2,10 +2,13 @@
 
 tests/emul/tb_emul.cpp compiles csrc/tb_*.cuh as plain C++ and runs one 32-lane warp of it as cooperative fibres.
 `Emul` is the single-env view the parity tests use; `EmulWarp` steps up to 10 envs in one warp, which exercises the
-predication of envs that need different numbers of Newton iterations / line-search evaluations / contacts."""
+predication of envs that need different numbers of Newton iterations / line-search evaluations / contacts.  Both run
+the per-env-parameter variant of the kernels when given parameter rows, the default variant otherwise."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -14,18 +17,26 @@ from tensegrity_rl_b200 import model as M
 HERE = os.path.dirname(os.path.abspath(__file__))
 STATE_STRIDE, INFO_DIM, HEADING_SLOTS, NDRAW = 96, 32, 32, 10
 EPW = 10
+NPARAM = 41
 _lib = None
 
 
-def lib(reverse=False):
+def lib():
+    """libtb_emul.so, compiled on first use into the temporary directory (the test tree may be read-only), under a
+    name that hashes the sources and flags it is built from"""
     global _lib
     if _lib is None:
-        so = os.path.join(HERE, "libtb_emul.so")
         csrc = os.path.join(os.path.dirname(os.path.dirname(HERE)), "tensegrity_rl_b200", "csrc")
-        deps = [os.path.join(HERE, "tb_emul.cpp")] + [os.path.join(csrc, f) for f in os.listdir(csrc) if f.startswith("tb_")]
-        if not os.path.isfile(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
-            subprocess.check_call(["g++", "-O2", "-fPIC", "-shared", "-std=c++17", "-ffp-contract=off",
-                                   "-Wno-unknown-pragmas", "-o", so, os.path.join(HERE, "tb_emul.cpp")])
+        src = os.path.join(HERE, "tb_emul.cpp")
+        cmd = ["g++", "-O2", "-fPIC", "-shared", "-std=c++17", "-ffp-contract=off", "-Wno-unknown-pragmas"]
+        h = hashlib.sha256(" ".join(cmd).encode())
+        for d in [src] + sorted(os.path.join(csrc, f) for f in os.listdir(csrc) if f.startswith("tb_")):
+            h.update(open(d, "rb").read())
+        so = os.path.join(tempfile.gettempdir(), "libtb_emul-%d-%s.so" % (os.getuid(), h.hexdigest()[:16]))
+        if not os.path.isfile(so):
+            tmp = "%s.%d.tmp" % (so, os.getpid())
+            subprocess.check_call(cmd + ["-o", tmp, src])
+            os.replace(tmp, so)      # whole files only, for concurrent test processes
         L = C.CDLL(so)
         L.tbe_create.restype = C.c_char_p
         assert L.tbe_envs_per_warp() == EPW
@@ -38,10 +49,14 @@ def P(a, t=C.c_double):
 
 
 class EmulWarp:
-    """n <= 10 envs stepped together by one emulated warp."""
+    """n <= 10 envs stepped together by one emulated warp.  With rows [n (+ pool slots)][41] the per-env variant runs:
+    the rows are kept and updated in place (self.params), as the device keeps d_params; prange [3][41] = nominal, lo,
+    hi of the reset draws (None = rows kept at resets)."""
 
-    def __init__(self, xml_file="flat", n=1, **env_kwargs):
+    def __init__(self, xml_file="flat", n=1, rows=None, prange=None, **env_kwargs):
         assert 1 <= n <= EPW
+        if prange is not None and rows is None:
+            raise ValueError("prange needs parameter rows")
         self.n = n
         self.md = M.load_model(xml_file)
         self.model, self._keep = M.model_struct(self.md)
@@ -59,6 +74,9 @@ class EmulWarp:
         self.draws = np.zeros((n, NDRAW))
         self.rec[:, 0:21] = self.md["qpos0"]
         self.real_obs = None
+        self.params = None if rows is None else np.ascontiguousarray(rows, np.float64)
+        self.prange = None if prange is None else np.ascontiguousarray(prange, np.float64)
+        self.L.tbe_set_params(self.h, P(self.params), P(self.prange))
 
     def __del__(self):
         try:
@@ -103,12 +121,17 @@ class EmulWarp:
         self.L.tbe_forward(self.h, self.n, P(self.rec), P(self.heading), P(self.obs), P(self.info))
         return self.obs.copy(), self.info.copy()
 
+    def pool(self, n_pool, rec, heading, draws, pool_obs, seed, finish_now=False):
+        """one pool advance over records [n + n_pool] (self.params, if set, then holds n + n_pool rows)"""
+        self.L.tbe_pool(self.h, self.n, int(n_pool), P(rec), P(heading), P(draws), P(pool_obs), C.c_ulonglong(seed),
+                        int(finish_now))
+
 
 class Emul:
-    """single env (the other 9 env slots of the warp idle)"""
+    """single env (the other 9 env slots of the warp idle), with its parameter row if one is given"""
 
-    def __init__(self, xml_file="flat", reverse=False, **env_kwargs):
-        self.w = EmulWarp(xml_file, 1, **env_kwargs)
+    def __init__(self, xml_file="flat", row=None, **env_kwargs):
+        self.w = EmulWarp(xml_file, 1, rows=None if row is None else np.asarray(row)[None, :], **env_kwargs)
         self.md, self.cfg, self.L = self.w.md, self.w.cfg, self.w.L
         self.rec = self.w.rec[0]
         self.heading = self.w.heading[0]
@@ -155,9 +178,25 @@ def reset_noise(seed, stream, nreset):
     return out[:21], out[21:]
 
 
-def obs_normals(seed, stream, nreset, step, n, reverse=False):
+def obs_normals(seed, stream, nreset, step, n):
     """the standard-normal draws the CUDA source uses for the observation of (stream, reset count, episode step)"""
     out = np.zeros(n + 1)
     lib().tbe_obs_normals(C.c_ulonglong(seed), C.c_ulonglong(stream), C.c_ulonglong(nreset), C.c_ulonglong(step),
                           int(n), P(out))
     return out[:n]
+
+
+def nominal_params(md):
+    """the nominal parameter row as the CUDA source builds it from the TsgModel struct"""
+    m, _keep = M.model_struct(md)
+    out = np.zeros(NPARAM)
+    lib().tbe_nominal_params(C.byref(m), P(out))
+    return out
+
+
+def param_draws(prange, seed, stream0, nreset, n=1):
+    """the parameter rows [n][41] that reset `nreset` of streams stream0 .. stream0 + n - 1 draws"""
+    pr = np.ascontiguousarray(prange, np.float64)
+    out = np.zeros((n, NPARAM))
+    lib().tbe_param_draws(P(out), P(pr), C.c_ulonglong(seed), C.c_ulonglong(stream0), C.c_ulonglong(nreset), int(n))
+    return out

@@ -7,7 +7,6 @@ import numpy as np
 import pytest
 
 from emul import emul as E
-from emul import emul_params as EP
 from oracle import oracle as O
 from oracle.envs import OracleEnv
 from tensegrity_rl_b200 import lib as tlib
@@ -27,7 +26,8 @@ def _random_rows(md, rng, n, lo=0.7, hi=1.3):
 
 def _warp_pair(xml, n, **kw):
     """the default variant and the per-env variant with nominal rows"""
-    return E.EmulWarp(xml, n, **kw), EP.EmulWarpP(xml, n, **kw)
+    rows = np.tile(E.nominal_params(M.load_model(xml)), (n, 1))
+    return E.EmulWarp(xml, n, **kw), E.EmulWarp(xml, n, rows=rows, **kw)
 
 
 def _oracle_env(xml, kind, row, **kw):
@@ -74,7 +74,7 @@ def test_distinct_rows_single_step_match_oracle(oracle, xml, pre):
     n = 10
     rng = np.random.default_rng(4)
     rows = _random_rows(M.load_model(xml), rng, n)
-    w = EP.EmulWarpP(xml, n, rows=rows)
+    w = E.EmulWarp(xml, n, rows=rows)
     mjs = [oracle.MjLike(xml, **M.param_overrides(r)) for r in rows]
     for i, mj in enumerate(mjs):
         for _ in range(pre + i):
@@ -110,7 +110,7 @@ def test_distinct_row_env_semantics_match_oracle_env(xml, kind, task):
     rng = np.random.default_rng(12)
     for trial in range(2):
         row = _random_rows(M.load_model(xml), rng, 1)[0]
-        em = EP.EmulP(xml, row, env_kind=kind, desired_action=task)
+        em = E.Emul(xml, row, env_kind=kind, desired_action=task)
         oe = _oracle_env(xml, kind, row, desired_action=task)
         d = _draws(rng, 1)[0]
         o1, o2 = oe.reset(d), em.reset(d)
@@ -135,12 +135,12 @@ def test_param_draws_keys_bounds_and_shared_lengthspring_draw():
     nom = M.nominal_params(md)
     lo, hi = M.param_scale_ranges({f: (0.8, 1.2) for f in tlib.PARAM})
     pr = _prange(md, lo, hi)
-    a, b = EP.param_draws(pr, 7, 3, 0), EP.param_draws(pr, 7, 3, 0)
+    a, b = E.param_draws(pr, 7, 3, 0), E.param_draws(pr, 7, 3, 0)
     assert np.array_equal(a, b)
-    for other in (EP.param_draws(pr, 8, 3, 0), EP.param_draws(pr, 7, 4, 0), EP.param_draws(pr, 7, 3, 1)):
+    for other in (E.param_draws(pr, 8, 3, 0), E.param_draws(pr, 7, 4, 0), E.param_draws(pr, 7, 3, 1)):
         assert not np.array_equal(a, other)
-    rows = EP.param_draws(pr, 1, 0, 0, n=4000)
-    assert np.array_equal(rows[5], EP.param_draws(pr, 1, 5, 0)[0])
+    rows = E.param_draws(pr, 1, 0, 0, n=4000)
+    assert np.array_equal(rows[5], E.param_draws(pr, 1, 5, 0)[0])
     lo_v, hi_v = np.minimum(nom * 0.8, nom * 1.2), np.maximum(nom * 0.8, nom * 1.2)
     assert ((rows >= lo_v) & (rows <= hi_v)).all()
     s = rows[:, nom != 0] / nom[nom != 0]
@@ -151,7 +151,7 @@ def test_param_draws_keys_bounds_and_shared_lengthspring_draw():
     assert not np.array_equal(ls[:, 0, 0], ls[:, 1, 0])            # ... and the tendons draw independently
     # lo == hi: exactly nominal * lo
     lo2 = np.full(41, 0.9); lo2[0] = 1.0
-    assert np.array_equal(EP.param_draws(_prange(md, lo2, lo2), 5, 9, 2, n=3), np.tile(nom * lo2, (3, 1)))
+    assert np.array_equal(E.param_draws(_prange(md, lo2, lo2), 5, 9, 2, n=3), np.tile(nom * lo2, (3, 1)))
 
 
 @pytest.mark.parametrize("noise", [False, True])
@@ -163,7 +163,7 @@ def test_reset_draws_rows_and_other_draws_unchanged(noise):
     md = M.load_model("flat")
     nom = M.nominal_params(md)
     pr1 = _prange(md, np.ones(41), np.ones(41))
-    a, b = E.EmulWarp("flat", n, **kw), EP.EmulWarpP("flat", n, rows=np.zeros((n, 41)), prange=pr1, **kw)
+    a, b = E.EmulWarp("flat", n, **kw), E.EmulWarp("flat", n, rows=np.zeros((n, 41)), prange=pr1, **kw)
     rows = b.params
     if noise:
         a.set_noise(seed, 100); b.set_noise(seed, 100)
@@ -177,12 +177,12 @@ def test_reset_draws_rows_and_other_draws_unchanged(noise):
     # ranges on: new rows, the same reset draws
     lo, hi = M.param_scale_ranges({f: (0.8, 1.2) for f in tlib.PARAM})
     pr = _prange(a.md, lo, hi)
-    c = EP.EmulWarpP("flat", n, rows=np.zeros((n, 41)), prange=pr, **kw)
+    c = E.EmulWarp("flat", n, rows=np.zeros((n, 41)), prange=pr, **kw)
     rows = c.params
     c.rec[:, 85] = 3          # reset count 3
     a.rec[:, 85] = 3
     c.reset(seed=seed, env_id=100); a.reset(seed=seed, env_id=100)
-    assert np.array_equal(rows, EP.param_draws(pr, seed, 100, 3, n=n))
+    assert np.array_equal(rows, E.param_draws(pr, seed, 100, 3, n=n))
     assert np.array_equal(a.draws, c.draws)
     d = np.zeros(10)
     E.lib().tbe_make_draws(E.P(d), C.c_ulonglong(seed), C.c_ulonglong(104), C.c_ulonglong(3))
@@ -194,13 +194,13 @@ def test_pool_slot_draws_its_row_at_phase_zero():
     md = M.load_model("flat")
     lo, hi = M.param_scale_ranges({"ten_stiffness": (0.5, 1.5), "act_gain": (0.9, 1.1)})
     pr = _prange(md, lo, hi)
-    w = EP.EmulWarpP("flat", n_envs, rows=np.tile(M.nominal_params(md), (n_envs + n_pool, 1)), prange=pr, warmup_steps=2)
+    w = E.EmulWarp("flat", n_envs, rows=np.tile(M.nominal_params(md), (n_envs + n_pool, 1)), prange=pr, warmup_steps=2)
     rows = w.params
     rec = np.zeros((n_envs + n_pool, 96)); rec[:, 0:21] = w.md["qpos0"]
     head = np.zeros((n_envs + n_pool, 32)); draws = np.zeros((n_envs + n_pool, 10))
     pool_obs = np.zeros((n_pool, w.cfg.obs_dim))
     w.pool(n_pool, rec, head, draws, pool_obs, seed)
-    assert np.array_equal(rows[n_envs:], EP.param_draws(pr, seed, 1 << 40, 0, n=n_pool))
+    assert np.array_equal(rows[n_envs:], E.param_draws(pr, seed, 1 << 40, 0, n=n_pool))
     assert np.array_equal(rows[:n_envs], np.tile(M.nominal_params(w.md), (n_envs, 1)))
     before = rows.copy()
     w.pool(n_pool, rec, head, draws, pool_obs, seed)
@@ -212,7 +212,7 @@ def test_nominal_params_match_model_struct():
     for xml in ("flat", "uneven"):
         md = M.load_model(xml)
         row = M.nominal_params(md)
-        assert np.array_equal(row, EP.nominal_params(md))
+        assert np.array_equal(row, E.nominal_params(md))
         ov = M.param_overrides(row)
         for k, v in ov.items():
             assert np.array_equal(np.asarray(v, float).reshape(-1), np.asarray(md[k], float).reshape(-1)), k

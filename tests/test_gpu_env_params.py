@@ -112,14 +112,14 @@ def test_reset_rows_equal_emulator_draws_and_shards_reproduce():
     """rows after reset_tensor() are the emulator's draws bit for bit; two handles with env_id_base reproduce one
     unsharded handle through auto resets (reset_pool=0)"""
     import torch
-    from emul import emul_params as EP
+    from emul import emul as E
     n, seed = 2048, 17
     kw = dict(seed=seed, reset_pool=0, max_episode_steps=8, param_ranges=RANGES)
     full = _vec(n, **kw)
     lo, hi = M.param_scale_ranges(RANGES)
     pr = np.stack([M.nominal_params(full.md), lo, hi])
     obs_full = [full.reset_tensor().cpu().numpy()]
-    assert np.array_equal(full.get_env_params().cpu().numpy(), EP.param_draws(pr, seed, 0, 0, n=n))
+    assert np.array_equal(full.get_env_params().cpu().numpy(), E.param_draws(pr, seed, 0, 0, n=n))
     shards = [_vec(n // 2, env_id_base=k * (n // 2), **kw) for k in range(2)]
     obs_sh = [np.concatenate([s.reset_tensor().cpu().numpy() for s in shards])]
     g = torch.Generator(device="cuda"); g.manual_seed(5)
@@ -135,7 +135,7 @@ def test_reset_rows_equal_emulator_draws_and_shards_reproduce():
     nres = full.get_records()[:, 85].astype(int)
     assert nres.min() >= 2         # every env was redrawn at its auto resets
     for e in (0, 1, n - 1):
-        assert np.array_equal(p_full[e], EP.param_draws(pr, seed, e, nres[e] - 1)[0])
+        assert np.array_equal(p_full[e], E.param_draws(pr, seed, e, nres[e] - 1)[0])
     for v in [full] + shards:
         v.close()
 
@@ -144,7 +144,7 @@ def test_pool_resets_hand_over_valid_draws(oracle):
     """with a reset pool every env that auto-reset holds a row a slot drew, and its next step matches the oracle
     built from that row"""
     import torch
-    from emul import emul_params as EP
+    from emul import emul as E
     n, seed = 1024, 23
     v = _vec(n, seed=seed, reset_pool="auto", max_episode_steps=6, param_ranges=RANGES)
     lo, hi = M.param_scale_ranges(RANGES)
@@ -152,8 +152,8 @@ def test_pool_resets_hand_over_valid_draws(oracle):
     v.reset_tensor()
     g = torch.Generator(device="cuda"); g.manual_seed(8)
     # a slot's draws, or (done envs that found no ready slot reset synchronously) the env's own
-    drawn = {r.tobytes() for k in range(4) for r in EP.param_draws(pr, seed, 1 << 40, k, n=v.reset_pool)}
-    drawn |= {r.tobytes() for k in range(4) for r in EP.param_draws(pr, seed, 0, k, n=n)}
+    drawn = {r.tobytes() for k in range(4) for r in E.param_draws(pr, seed, 1 << 40, k, n=v.reset_pool)}
+    drawn |= {r.tobytes() for k in range(4) for r in E.param_draws(pr, seed, 0, k, n=n)}
     assigned, nbad, ncheck = 0, 0, 0
     for st in range(14):
         a = -0.45 + 0.6 * torch.rand(n, 6, generator=g, device="cuda", dtype=torch.float64)

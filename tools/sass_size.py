@@ -3,7 +3,7 @@
 usage: sass_size.py DIS [KERNEL]
   DIS     `nvdisasm -gi` output of the library's cubin (tools/README.md)
   KERNEL  substring of the mangled kernel name; default: the step kernel (MODE = 0) of the production shape,
-          tb_env_kernel<P64, 0, 6, 10>
+          tb_env_kernel<P64, 0, 6>
 
 Every instruction carries its inline chain, innermost source line first.  Each source line is mapped to the TB_FN /
 TB_NOINL / __global__ function of csrc/ whose definition precedes it.  `self` counts an instruction for the innermost
@@ -48,7 +48,7 @@ def device_function(symbol):
 
 def main():
     dis = sys.argv[1]
-    want = sys.argv[2] if len(sys.argv) > 2 else "tb_env_kernelIN2tb3P64ELi0ELi6ELi10E"
+    want = sys.argv[2] if len(sys.argv) > 2 else "tb_env_kernelIN2tb3P64ELi0ELi6EEv"
     defs = definitions()
     loc = re.compile(r'//## File "([^"]+)", line (\d+)(?: inlined at "([^"]+)", line (\d+))?')
     sec, dev, chain = None, None, []
